@@ -10,12 +10,15 @@ object's 4096 candidates; step k works on object k mod 8, so K >= 8 steps cover 
 for the Allegro and LEAP hands (configs[3]).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--workload robotiq|panda|allegro|leap|mixed|clutter_shadow]
+                  [--workload robotiq|panda|allegro|leap|mixed|clutter_shadow] [--dump-outputs DIR]
 
   value  = env-steps/s with inputs resident in HBM, timed with CUDA events on the launch stream
   e2e    = the same metric through the host-pointer C-ABI call (pinned H2D + kernel + D2H inside the call)
   --impl reference = the CPU arm: the fp64 oracle port (MuJoCo is not installable here) on all host threads, on a bounded
            sample of the SAME candidate sets.
+  --dump-outputs DIR = after the run, DIR/<line>_labels.npy and DIR/<line>_steps.npy (float32, one value per candidate) hold what
+           the last timed step of each line of the JSON result returned (<line> = the workload, or its name under "also"; the
+           mixed batch returns labels only, in bucket order).  The inputs are seeded, so two builds can be compared file by file.
 
 Multi-GPU (torchrun, one rank per GPU): robotiq / panda / hands are WEAK scaling - every rank runs the same object sequence, so
 a loss of efficiency is the machine's, not a difference in work; `per_rank` holds every rank's kernel time.  `--workload mixed`
@@ -165,6 +168,15 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(path, outputs):
+    """outputs: {line: {array name: per-candidate array}} -> path/<line>_<array name>.npy in float32 (labels are 0 / 1, step
+    counts stay below 2^24, so float32 holds both exactly)."""
+    os.makedirs(path, exist_ok=True)
+    for line, arrays in outputs.items():
+        for name, a in arrays.items():
+            np.save(os.path.join(path, f"{line}_{name}.npy"), np.asarray(a, dtype=np.float32))
+
+
 def load_json(*path):
     try:
         return json.load(open(os.path.join(ROOT, *path)))
@@ -193,6 +205,7 @@ def run_ours(args, rank, world, local_rank):
     # phase (tools/ncu_summary.py --json) - both derived by committed scripts from ncu captures, nothing typed in here
     traffic = load_json("profiles", "traffic_r2.json") or load_json("profiles", "traffic_r1.json")
     issue = load_json("profiles", "issue_slots_r2.json")
+    outputs = {} if args.dump_outputs else None  # line -> arrays of its last timed step (--dump-outputs)
 
     def barrier():
         if dist is not None:
@@ -232,9 +245,10 @@ def run_ours(args, rank, world, local_rank):
                 "peak_ginst_s": peak_issue / 1e9, "frac": ipe * value_per_gpu / peak_issue}
 
     # ------------------------------------------------------------------------------------------------ single-model workloads
-    def measure(key, steps, warmup, with_cpu):
+    def measure(key, steps, warmup, with_cpu, line=None):
         """W warm-up + K timed passes on device-resident inputs (CUDA events), then K passes through the host-pointer C ABI.
-        Step k works on object k mod n_objects.  Returns the JSON fields of that workload (rank 0) or None."""
+        Step k works on object k mod n_objects.  Returns the JSON fields of that workload (rank 0) or None.  `line`: the name
+        of its outputs (default: key)."""
         W = WORKLOADS[key]
         gripper = W["gripper"]
         N_CAND = W.get("n", 4096)
@@ -281,6 +295,8 @@ def run_ours(args, rank, world, local_rank):
                 overflowed += sets[k % nobj]["sim"].overflow_count()
             barrier()
             t_wall = time.perf_counter() - t_begin
+        if outputs is not None:
+            outputs[line or key] = dict(labels=d_lab.cpu().numpy(), steps=d_steps.cpu().numpy())
         launches = sum(gather_ranks(L.mgs_launch_count() - launches0))
         dev_s = sum(kern_ms) / 1e3
         # end-to-end through the host-pointer C ABI (pinned staging, H2D + kernel + D2H inside the call)
@@ -401,6 +417,8 @@ def run_ours(args, rank, world, local_rank):
                 stable += int(sum(l.sum() for l in labels))
             barrier()
             t_wall = time.perf_counter() - t_begin
+        if outputs is not None:
+            outputs["mixed"] = dict(labels=np.concatenate(labels))
         launches = sum(gather_ranks(lib.mgs_launch_count() - launches0))
         host[0] = True
         barrier()
@@ -442,7 +460,7 @@ def run_ours(args, rank, world, local_rank):
         import clutter_shadow_bench as csb
         return csb.measure(args, rank, world, local_rank, steps, warmup, with_cpu, dict(
             torch=torch, dist=dist, dev=dev, flush=flush, stream=stream, barrier=barrier, gather_ranks=gather_ranks, per_rank_block=per_rank_block,
-            roofline=roofline, ClockSampler=ClockSampler, desc=CLUTTER_DESC, cpu_arm=None))
+            roofline=roofline, ClockSampler=ClockSampler, desc=CLUTTER_DESC, cpu_arm=None, outputs=outputs))
 
     with_cpu = world == 1 and not args.no_cpu
     if args.workload == "mixed":
@@ -459,7 +477,7 @@ def run_ours(args, rank, world, local_rank):
         if world == 1 and not args.no_hands:
             side += [("allegro", "allegro", 1, 2, False), ("leap", "leap", 1, 2, False)]
         for name, key, k, w, cpu in side:
-            r = measure(key, k, w, cpu)
+            r = measure(key, k, w, cpu, line=name)
             if rank == 0:
                 also[name] = {q: r[q] for q in ("value", "unit", "steps", "warmup", "ms_per_step", "grasps_per_s", "dtype", "e2e", "config", "roofline", "issue_slots",
                                                   "gpu_launches", "per_rank", "cpu_baseline") if q in r}
@@ -467,6 +485,8 @@ def run_ours(args, rank, world, local_rank):
         if also:
             line["also"] = also
             line["gpu_launches"] += sum(a["gpu_launches"] for a in also.values())
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -483,7 +503,13 @@ def main():
     ap.add_argument("--no-hands", action="store_true", help="skip the Allegro / LEAP lines")
     ap.add_argument("--caps", default="", help="override the primary workload's per-environment capacities: ncon_max,nefc_max")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the labels and step counts of each line's last timed step to DIR/<line>_<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the CPU arm evaluates a time-bounded sample, not a fixed set)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -2,6 +2,7 @@
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 from mj_grasp_sim_b200 import lib as mlib
 
@@ -13,9 +14,17 @@ def build(f64=False):
     so = os.path.join(_HERE, "liblane1_f64.so" if f64 else "liblane1_f32.so")
     srcs = [os.path.join(_HERE, "lane1.cpp")] + mlib._sources()
     if not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(s) for s in srcs):
-        cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared"] + (["-DMGS_REAL_DOUBLE"] if f64 else []) + [
-            "-x", "c++", "-o", so, os.path.join(_HERE, "lane1.cpp")]
-        subprocess.check_call(cmd)
+        # compile to a private file and rename it into place: parallel test workers never load a half-written library
+        fd, tmp = tempfile.mkstemp(suffix=".so", dir=_HERE)
+        os.close(fd)
+        try:
+            cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared"] + (["-DMGS_REAL_DOUBLE"] if f64 else []) + [
+                "-x", "c++", "-o", tmp, os.path.join(_HERE, "lane1.cpp")]
+            subprocess.check_call(cmd)
+            os.replace(tmp, so)
+        finally:
+            if os.path.exists(tmp):
+                os.remove(tmp)
     return so
 
 

@@ -382,7 +382,13 @@ def test_loaded_library_is_head_and_not_the_host_proxy(libs):
         assert mlib.load(f64=True).mgs_build_stamp().decode() == mlib.source_stamp()
     assert mlib.BatchSim.__module__ == "mj_grasp_sim_b200.lib" and mlib.BatchSim.__name__ == "BatchSim"
     assert "hostsim.lane1" not in sys.modules or os.environ.get("MGS_PROXY") is None
-    maps = open("/proc/self/maps").read()
+    assert "libmgs_b200.so" in open("/proc/self/maps").read()
+    # the CPU tier of the same pytest run may have mapped the host build here on purpose, so the absence of the host build is
+    # checked in a fresh interpreter with this environment (where the proxy would load it at start-up) that loads the library
+    import subprocess
+    probe = "import sys; sys.path.insert(0, sys.argv[1]); from mj_grasp_sim_b200 import lib; lib.load(); print(open('/proc/self/maps').read())"
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    maps = subprocess.run([sys.executable, "-c", probe, root], capture_output=True, text=True, check=True).stdout
     assert "libmgs_b200.so" in maps and "liblane1" not in maps
 
 

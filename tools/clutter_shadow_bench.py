@@ -87,6 +87,8 @@ def measure(args, rank, world, local_rank, steps, warmup, with_cpu, ctx):
             overflowed += sim.overflow_count()
         ctx["barrier"]()
         t_wall = time.perf_counter() - t_begin
+    if ctx["outputs"] is not None:
+        ctx["outputs"]["clutter_shadow"] = dict(labels=d_lab.cpu().numpy(), steps=d_steps.cpu().numpy())
     launches = sum(ctx["gather_ranks"](L.mgs_launch_count() - launches0))
     dev_s = sum(kern_ms) / 1e3
     ctx["barrier"]()
