@@ -44,7 +44,8 @@ typedef struct MgsRolloutCfg {
 } MgsRolloutCfg;
 
 typedef struct MgsModelInfo {
-  int nq, nv, nu, nmocap, state_stride, diag_stride, ncon_max, nefc_max, smem_bytes_per_env,
+  int nq, nv, nu, nmocap, state_stride, diag_stride, ncon_max, nefc_max,
+      smem_bytes_per_env, /* size of one environment's state: shared memory, or global memory when mgs_model_state_in_global() is 1 */
       warps_per_block, /* environments per CTA */
       blocks_per_sm, num_sms, real_bytes,
       lanes_per_env; /* threads that share one environment: 32 (warp per environment) or 256 (environment per CTA) */
@@ -55,6 +56,13 @@ int mgs_model_create(const MgsModelDesc *desc, int device, MgsModel **out);
  * pairs - 32 for models with more than 24 dofs - and static rows + 4 rows per contact slot).  Shared memory per environment - and so the number of environments resident per SM - follows
  * from them.  Contacts beyond capacity are dropped and counted in the diagnostics' overflow field. */
 int mgs_model_create_ex(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, MgsModel **out);
+/* Same as mgs_model_create_ex (same kernel selection, same capacities), except that a model whose environment state does not fit one
+ * CTA's shared memory - where _ex fails - is created on the environment-per-CTA variant with the state in a global-memory slab
+ * (one slice per CTA of the persistent grid, allocated here, freed by mgs_model_destroy).  mgs_model_create / _ex keep failing
+ * there, so a caller can still probe for the largest capacity that fits shared memory. */
+int mgs_model_create_any(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, MgsModel **out);
+/* 1: the model's environment state lives in global memory (variant wide_g), 0: in shared memory, <0: error */
+int mgs_model_state_in_global(const MgsModel *model);
 void mgs_model_destroy(MgsModel *model);
 int mgs_model_info(const MgsModel *model, MgsModelInfo *info);
 

@@ -56,6 +56,7 @@ struct MgsModel {
   int aux_cap, aux_n;
   double qvel_clip;
   cudaStream_t stream;
+  real *d_env_state;  // wide_g variant: the environments' state, one Layout.total slice per CTA of the persistent grid (else null)
 };
 
 extern "C" const char *mgs_last_error(void) { return g_err.c_str(); }
@@ -66,7 +67,10 @@ extern "C" int mgs_model_create(const MgsModelDesc *desc, int device, MgsModel *
   return mgs_model_create_ex(desc, device, 0, 0, out);
 }
 
-extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, MgsModel **out) {
+// allow_global: a model whose environment state does not fit one CTA's shared memory runs on the wide_g variant (state in a global
+// slab) instead of failing - mgs_model_create_any.  mgs_model_create / _ex keep failing there: callers (EscalatingSim) probe for the
+// largest capacity that fits shared memory that way.
+static int model_create(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, bool allow_global, MgsModel **out) {
   if (!desc || !out) return fail("null argument");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("no CUDA device: libmgs_b200 has no CPU path");
@@ -107,7 +111,8 @@ extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int nco
   // MGS_WIDE_BELOW_ENVS environments per SM (or for none) run the environment-per-CTA variant instead.
   const char *force_wpb = getenv("MGS_WARPS_PER_BLOCK");  // tuning knobs: force the CTA size / the variant
   const char *force_var = getenv("MGS_KERNEL_VARIANT");
-  const bool force_wide = force_var && std::string(force_var) == "wide";
+  const bool force_wide_g = force_var && std::string(force_var) == "wide_g";
+  const bool force_wide = (force_var && std::string(force_var) == "wide") || force_wide_g;
   std::lock_guard<std::mutex> lock(g_launch_mu);  // the occupancy sweep changes the variants' shared-memory attribute
   const MgsKernelOps *variants[2] = {mgs_kernel_ops_w16(), mgs_kernel_ops_w12()};
   int best_warps = 0;
@@ -155,16 +160,20 @@ extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int nco
     ncache_max = MGS_MPR_CACHE_MAX;
     env_bytes = make_layout(32);
   }
+  bool in_global = false;
   if (force_wide || (!force_var && best_warps < MGS_WIDE_BELOW_ENVS)) {
     const MgsKernelOps *ops = mgs_kernel_ops_wide();
     env_bytes = make_layout(ops->lanes_per_env);
-    if ((size_t)env_bytes > prop.sharedMemPerBlockOptin) {
+    in_global = force_wide_g || (allow_global && (size_t)env_bytes > prop.sharedMemPerBlockOptin);
+    if (in_global) ops = mgs_kernel_ops_wide_g();  // same lanes per environment, so the same layout
+    if (!in_global && (size_t)env_bytes > prop.sharedMemPerBlockOptin) {
       delete M;
       return fail("model needs more shared memory per environment than one CTA can have: lower ncon_max / nefc_max");
     }
-    CU(ops->prepare(env_bytes));
+    const int dyn_smem = in_global ? 0 : env_bytes;
+    CU(ops->prepare(dyn_smem));
     int occ = 0;
-    CU(ops->occupancy(&occ, ops->lanes_per_env, (size_t)env_bytes));
+    CU(ops->occupancy(&occ, ops->lanes_per_env, (size_t)dyn_smem));
     best_warps = occ;
     M->warps_per_block = 1; M->blocks_per_sm = occ; M->ops = ops;
   }
@@ -174,7 +183,16 @@ extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int nco
     CU(cudaMalloc(&M->d_mpr_cache, slots * desc->npair * 4 * sizeof(int)));
   }
   if (best_warps == 0) { delete M; return fail("kernel does not fit on this device"); }
-  M->smem_per_block = env_bytes * M->warps_per_block;
+  if (in_global) {  // one slice per CTA of the persistent grid (launch() never starts more CTAs than that)
+    const size_t slab = (size_t)M->num_sms * M->blocks_per_sm * env_bytes;
+    if (cudaMalloc(&M->d_env_state, slab) != cudaSuccess) {
+      cudaGetLastError();
+      M->d_env_state = nullptr;
+      mgs_model_destroy(M);
+      return fail("cannot allocate the global-memory environment state (" + std::to_string(slab >> 20) + " MiB)");
+    }
+  }
+  M->smem_per_block = in_global ? 0 : env_bytes * M->warps_per_block;
   // (the attribute is set again before every launch: it belongs to the kernel function, not to this model)
   M->state_stride = desc->nq + 2 * desc->nv + desc->nu + 7 * desc->nmocap;
   M->diag_stride = mgs_diag_stride(desc->nv, desc->nbody, blob.ncon_max, blob.nefc_max);
@@ -183,12 +201,26 @@ extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int nco
   return 0;
 }
 
+extern "C" int mgs_model_create_ex(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, MgsModel **out) {
+  return model_create(desc, device, ncon_max, nefc_max, false, out);
+}
+
+extern "C" int mgs_model_create_any(const MgsModelDesc *desc, int device, int ncon_max, int nefc_max, MgsModel **out) {
+  return model_create(desc, device, ncon_max, nefc_max, true, out);
+}
+
+extern "C" int mgs_model_state_in_global(const MgsModel *M) {
+  if (!M) return fail("null model");
+  return M->d_env_state ? 1 : 0;
+}
+
 extern "C" void mgs_model_destroy(MgsModel *M) {
   if (!M) return;
   cudaSetDevice(M->device);
   cudaFree(M->d_blob);
   cudaFree(M->d_counter);
   if (M->d_mpr_cache) cudaFree(M->d_mpr_cache);
+  if (M->d_env_state) cudaFree(M->d_env_state);
   if (M->d_aux) cudaFree(M->d_aux);
   if (M->d_stage) cudaFree(M->d_stage);
   if (M->h_stage) cudaFreeHost(M->h_stage);
@@ -247,6 +279,7 @@ static int launch(MgsModel *M, const RolloutParams &prm, const BatchIO &io_in, c
   }
   io.aux = M->d_aux;
   io.mpr_cache_g = M->d_mpr_cache;
+  io.env_state = M->d_env_state;
   M->aux_n = prm.n;
   // Wave quantisation: every candidate of a batch costs about the same, so what matters is the number of
   // "waves" of resident environments.  If fewer warps per CTA give the same number of waves, use fewer: each

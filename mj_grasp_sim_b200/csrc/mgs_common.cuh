@@ -234,4 +234,8 @@ struct BatchIO {
   // per-pair MPR cache of the pairs beyond the shared-memory one (4 words per pair, one slab of npair pairs per environment slot of the
   // persistent grid; L2 resident) - null for models whose pairs all fit the shared-memory cache
   int *mpr_cache_g;
+  // environment-per-CTA variant with the state in global memory (csrc/mgs_kernel_wide_g.cu): one Layout.total slice per CTA of the
+  // persistent grid - null for the variants that keep it in shared memory.  Last member: the constant-bank offsets of the fields
+  // above stay where they were.
+  real *env_state;
 };

@@ -1,5 +1,6 @@
 // mgs_kernel.cuh - the persistent rollout kernel, instantiated once per translation unit.
-// Expects MGS_KERNEL_TAG (w16, w12) and MGS_MAX_WARPS_PER_BLOCK to be defined by the including .cu file.
+// Expects MGS_KERNEL_TAG (w16, w12, wide, wide_g) and MGS_MAX_WARPS_PER_BLOCK to be defined by the including .cu file (MGS_WIDE for
+// the environment-per-CTA variants, MGS_ENV_GLOBAL for the one whose environment state lives in global memory).
 //
 // Launch shape: a persistent grid of (blocks_per_sm x 148) CTAs, each up to MGS_MAX_WARPS_PER_BLOCK warps; every warp
 // pulls candidate indices from a global atomic work queue, so warps that finish early (candidates that fail the
@@ -18,7 +19,11 @@
 __global__ void __launch_bounds__(MGS_WIDE, 1)
 MGS_KERNEL() {
   __shared__ unsigned int s_env;
+#ifdef MGS_ENV_GLOBAL
+  real *base = IO.env_state + (size_t)blockIdx.x * LY.total;
+#else
   real *base = reinterpret_cast<real *>(mgs_smem_raw);
+#endif
   Env e;
   for (;;) {
     if (threadIdx.x == 0) s_env = atomicAdd(IO.work_counter, 1u);
@@ -50,11 +55,23 @@ MGS_KERNEL() {
 #endif
 
 namespace {
+#ifdef MGS_ENV_GLOBAL
+// No dynamic shared memory (the environment's state is in the global slab): the carveout goes to L1, which caches the slab.
+// MGS_CARVEOUT=default keeps the driver's choice instead (A/B knob).
+cudaError_t ops_prepare(int) {
+  const char *c = getenv("MGS_CARVEOUT");
+  const int carveout = (c && std::string(c) == "default") ? (int)cudaSharedmemCarveoutDefault : (int)cudaSharedmemCarveoutMaxL1;
+  cudaError_t rc = cudaFuncSetAttribute(MGS_KERNEL, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
+  if (rc != cudaSuccess) return rc;
+  return cudaFuncSetAttribute(MGS_KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, 0);
+}
+#else
 cudaError_t ops_prepare(int smem_bytes) {
   cudaError_t rc = cudaFuncSetAttribute(MGS_KERNEL, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (rc != cudaSuccess) return rc;
   return cudaFuncSetAttribute(MGS_KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
 }
+#endif
 cudaError_t ops_occupancy(int *blocks_per_sm, int threads, size_t smem_bytes) {
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, MGS_KERNEL, threads, smem_bytes);
 }

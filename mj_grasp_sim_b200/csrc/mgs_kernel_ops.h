@@ -23,4 +23,7 @@ const MgsKernelOps *mgs_kernel_ops_w12();
 // environment per CTA (csrc/mgs_kernel_wide.cu): scenes whose state leaves room for fewer than MGS_WIDE_BELOW_ENVS
 // warp-environments per SM (Shadow hand in 10-object clutter: one)
 const MgsKernelOps *mgs_kernel_ops_wide();
+// the same with the environment's state in a global-memory slab (csrc/mgs_kernel_wide_g.cu): scenes whose state does not fit one CTA's
+// shared memory at all (fp64 Shadow hand over four or more clutter objects, clutter escalation capacities); mgs_model_create_any only
+const MgsKernelOps *mgs_kernel_ops_wide_g();
 #define MGS_WIDE_BELOW_ENVS 4

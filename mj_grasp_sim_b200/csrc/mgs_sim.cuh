@@ -267,7 +267,13 @@ struct Env { real *base; };
 #define EBASE (e.base)
 #else
 extern __shared__ __align__(16) unsigned char mgs_smem_raw[];
-#ifdef MGS_WIDE
+#if defined(MGS_WIDE) && defined(MGS_ENV_GLOBAL)
+// environment per CTA with the slice in a global-memory slab (one slice per CTA of the persistent grid, BatchIO.env_state): scenes
+// whose state does not fit one CTA's shared memory.  Every access to the slice is a plain (coherent) load or store - nothing reads it
+// through LDG / __ldg - and WSYNC = __syncthreads() orders global memory within the CTA as it does shared memory, so no fence is needed.
+#define EBASE (IO.env_state + (size_t)blockIdx.x * LY.total)
+#define MGS_ENV_SLOT ((int)blockIdx.x)
+#elif defined(MGS_WIDE)
 #define EBASE (reinterpret_cast<real *>(mgs_smem_raw))
 #define MGS_ENV_SLOT ((int)blockIdx.x)  // index of this environment slot in the persistent grid
 #else

@@ -65,11 +65,12 @@ def build(force: bool = False, f64: bool = False) -> str:
     stamp = source_stamp()
     if not force and os.path.exists(so) and _built_stamp(so) == stamp:
         return so
-    # three translation units = three variants of the rollout kernel (16 / 12 warps per CTA with one environment per warp,
-    # and one environment per 256-thread CTA; see csrc/mgs_kernel_ops.h)
+    # four translation units = four variants of the rollout kernel (16 / 12 warps per CTA with one environment per warp, and one
+    # environment per 256-thread CTA with its state in shared or in global memory; see csrc/mgs_kernel_ops.h)
     cmd = ["nvcc"] + NVCC_FLAGS + (["-DMGS_REAL_DOUBLE"] if f64 else []) + [f'-DMGS_BUILD_STAMP="{stamp}"', "-o", so,
                                                                              os.path.join(CSRC, "mgs_b200.cu"), os.path.join(CSRC, "mgs_kernel_w12.cu"),
-                                                                             os.path.join(CSRC, "mgs_kernel_wide.cu"), os.path.join(CSRC, "mgs_sampler.cu")]
+                                                                             os.path.join(CSRC, "mgs_kernel_wide.cu"), os.path.join(CSRC, "mgs_kernel_wide_g.cu"),
+                                                                             os.path.join(CSRC, "mgs_sampler.cu")]
     subprocess.check_call(cmd)
     with open(so + ".stamp", "w") as f:
         f.write(stamp)
@@ -90,6 +91,8 @@ def bind(L, prefix="mgs_"):
     if prefix == "mgs_":
         L.mgs_model_create.argtypes = [C.POINTER(MgsModelDesc), C.c_int, C.POINTER(vp)]
         L.mgs_model_create_ex.argtypes = [C.POINTER(MgsModelDesc), C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
+        L.mgs_model_create_any.argtypes = [C.POINTER(MgsModelDesc), C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
+        L.mgs_model_state_in_global.argtypes = [vp]
         L.mgs_grasp_collision_mask.argtypes = [vp, C.c_int, fp, fp, C.c_int, ip, C.c_int, u8p]
         L.mgs_grasp_stability.argtypes = [vp, C.c_int, fp, fp, C.c_int, ip, C.c_int, dp, C.POINTER(MgsRolloutCfg), u8p, ip]
         L.mgs_rollout_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, C.c_int, ip, C.c_int, dp, C.POINTER(MgsRolloutCfg), vp, vp, vp]
@@ -131,10 +134,13 @@ class BatchSim:
 
     `lib`/`prefix` exist so the test tier can drive the lane-1 host build of the same source
     through the same wrapper; product code always uses the defaults (the CUDA library).
+
+    `global_fallback=True` (mgs_model_create_any): a model whose environment state does not fit one CTA's shared memory runs with
+    that state in global memory (kernel variant wide_g) instead of raising; `state_in_global` tells which one was made.
     """
 
     def __init__(self, model, device: int = 0, f64: bool = False, lib=None, prefix: str = "mgs_", ncon_max: int = 0, nefc_max: int = 0,
-                 ground_name: str = "geom:ground"):
+                 ground_name: str = "geom:ground", global_fallback: bool = False):
         self.model = model
         self.device = device
         self.L = lib if lib is not None else load(f64)
@@ -144,7 +150,8 @@ class BatchSim:
         if prefix == "mgs_":
             ncon_max = ncon_max or int(os.environ.get("MGS_NCON_MAX", "0"))
             nefc_max = nefc_max or int(os.environ.get("MGS_NEFC_MAX", "0"))
-            rc = self.L.mgs_model_create_ex(C.byref(self.desc), device, ncon_max, nefc_max, C.byref(h))
+            create = self.L.mgs_model_create_any if global_fallback else self.L.mgs_model_create_ex
+            rc = create(C.byref(self.desc), device, ncon_max, nefc_max, C.byref(h))
         else:
             rc = self.L.l1_model_create(C.byref(self.desc), C.byref(h))
         self._check(rc)
@@ -154,6 +161,16 @@ class BatchSim:
         self.real = np.float32 if self.info.real_bytes == 4 else np.float64
 
     def _f(self, name): return getattr(self.L, self.p + name)
+
+    @property
+    def state_in_global(self) -> bool:
+        """True when the environments' state lives in a global-memory slab (variant wide_g), False when in shared memory."""
+        if self.p != "mgs_":
+            return False
+        rc = self.L.mgs_model_state_in_global(self.h)
+        if rc < 0:
+            self._check(rc)
+        return bool(rc)
 
     def _check(self, rc):
         if rc != 0:

@@ -76,6 +76,14 @@ class MjSimulation:
     _device = None
     _caps = (0, 0)
     gripper = None
+    # True: a model whose environment state does not fit one CTA's shared memory keeps that state in global memory (kernel variant
+    # wide_g) instead of failing at creation (BatchSim(global_fallback=True)).  Set by ClutterTableEnv, whose fp64 Shadow-hand scenes
+    # and escalation capacities need it.
+    GLOBAL_STATE_FALLBACK = False
+
+    def _sim_kwargs(self) -> dict:
+        # passed only when set, so that a BatchSim stand-in without the argument keeps working for the other environments
+        return {"global_fallback": True} if self.GLOBAL_STATE_FALLBACK else {}
 
     @property
     def compute_f64(self) -> bool:
@@ -95,7 +103,7 @@ class MjSimulation:
                 import torch
                 dev = torch.cuda.current_device() if torch.cuda.is_available() else 0
             self._sim = BatchSim(self.model, device=dev, ncon_max=self._caps[0], nefc_max=self._caps[1], ground_name=self.GROUND_GEOM,
-                                 f64=self.compute_f64)
+                                 f64=self.compute_f64, **self._sim_kwargs())
         return self._sim
 
     # ---- single-environment state -------------------------------------------------------------

@@ -43,12 +43,15 @@ class ClutterTableEnv(MjSimulation):
         self._init_state()
 
     GROUND_GEOM = "geom:table"
+    # the fp64 Shadow hand over four or more objects, and the 256-contact escalation rung of every clutter scene, do not fit one
+    # CTA's shared memory: those models keep their environment state in global memory
+    GLOBAL_STATE_FALLBACK = True
 
     def _make_sim(self, caps):
         if caps is None:
             return self.sim
         return BatchSim(self.model, device=self.sim.device, ncon_max=caps[0], nefc_max=caps[1], ground_name=self.GROUND_GEOM,
-                        f64=self.compute_f64)
+                        f64=self.compute_f64, **self._sim_kwargs())
 
     @property
     def last_overflow(self):

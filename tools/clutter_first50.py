@@ -1,5 +1,7 @@
 """Config 5: qpos / qvel of the environment-per-CTA kernel vs the oracle over the first 50 steps after the hand is placed over the
-settled 10-object scene and told to close (8 candidates).  GPU box: python tools/clutter_first50.py"""
+settled 10-object scene and told to close (8 candidates).  fp32 (default): 80 contacts, state in shared memory; f64: the product
+path of ClutterTableEnv with the Shadow hand - default capacity, state in global memory.
+On a B200: python tools/clutter_first50.py [f32|f64]"""
 import os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -10,10 +12,14 @@ from oracle import oracle as orc
 import clutter_shadow_bench as csb
 
 
-def run(n=8, nstep=50, every=10, collision_free=True):
+def run(n=8, nstep=50, every=10, collision_free=True, f64=False):
     m, info = scenes.build_clutter_scene("shadow", list(range(10)))
-    G = BatchSim(m, ground_name="geom:table", ncon_max=csb.NCON_MAX)
-    step_fn = lambda r, k: G.step(r[None].astype(np.float32), k)[0].astype(np.float64)
+    if f64:
+        G = BatchSim(m, ground_name="geom:table", f64=True, global_fallback=True)
+    else:
+        G = BatchSim(m, ground_name="geom:table", ncon_max=csb.NCON_MAX)
+    print(f"{'fp64' if f64 else 'fp32'}, {G.info.ncon_max} contacts, state in {'global' if G.state_in_global else 'shared'} memory", flush=True)
+    step_fn = lambda r, k: G.step(r[None].astype(G.real), k)[0].astype(np.float64)
     rec = scenes.gen_clutter(m, info, step_fn, 7)
     pose7, joints = csb.make_inputs(scenes, m, info, rec, 16 * n)
     free = G.clutter_collision_mask(rec, pose7, joints, info["joint_qposadr"], info["base_qposadr"])
@@ -34,7 +40,7 @@ def run(n=8, nstep=50, every=10, collision_free=True):
     free = G.clutter_collision_mask(rec, pose7, joints, info["joint_qposadr"], info["base_qposadr"])
     print("collision-free at placement:", free.astype(int), flush=True)
     out = []
-    cur = st.astype(np.float32)
+    cur = st.astype(G.real)
     ref = [st[i].copy() for i in range(n)]
     for t in range(every, nstep + 1, every):
         cur, d = G.step(cur, every, want_diag=True)
@@ -54,4 +60,4 @@ def run(n=8, nstep=50, every=10, collision_free=True):
 
 
 if __name__ == "__main__":
-    run()
+    run(f64=len(sys.argv) > 1 and sys.argv[1] == "f64")
