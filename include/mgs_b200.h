@@ -100,6 +100,30 @@ int mgs_clutter_device(MgsModel *model, int mode, int n, const void *d_scene, co
                        const int *joint_qposadr, int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg,
                        uint8_t *d_labels, int *d_steps, void *stream);
 
+/* Many scenes of one model in one launch.  `scenes` holds nscene state records back to back ([nscene][state_stride]); candidate i
+ * starts from scene scene_index[i].  The plain variants reject an index outside [0, nscene); the device variant cannot check on the
+ * host, so such a candidate gets label 0, 0 steps and aux flag bit 1, and nothing is read at that index.  d_scene_index may be NULL
+ * (every candidate uses scene 0).  mgs_clutter_device is the nscene = 1, no-index, no-early-stop case of the same launch.
+ *
+ * enough_stable > 0 switches on the early stop of the reference's loop per scene (ClutterTableEnv.grasp_stable_mask, :293-296): the
+ * launch counts, per scene, the candidates that finished with label 1 and no capacity overflow; a candidate whose scene already
+ * counts >= enough_stable when it is pulled from the work queue is not simulated (label 0, 0 steps, aux flag bit 2).  Candidates are
+ * pulled in index order, so when each scene's candidates are in that scene's sequential order, a skipped candidate is one the
+ * sequential loop labels False; the others get their true label.  The caller still applies the prefix rule per scene (after
+ * re-running overflowed candidates at larger capacities): candidates after a scene's enough_stable-th success that were not
+ * skipped - they were in flight when the count was reached - keep their true label here.  Ordering candidates round-robin across
+ * scenes keeps that waste small.  The counters belong to the model (zeroed on the launch stream before every launch). */
+int mgs_clutter_scenes_collision_mask(MgsModel *model, int n, int nscene, const double *scenes, const int *scene_index,
+                                      const float *pose7, const float *joints, int nj, const int *joint_qposadr, int base_qposadr,
+                                      uint8_t *collision_free_out);
+int mgs_clutter_scenes_stable_mask(MgsModel *model, int n, int nscene, const double *scenes, const int *scene_index, const float *pose7,
+                                   const float *joints, int nj, const int *joint_qposadr, int base_qposadr, int enough_stable,
+                                   const double *close_ctrl, const MgsRolloutCfg *cfg, uint8_t *stable_out, int *steps_out);
+int mgs_clutter_scenes_device(MgsModel *model, int mode, int n, int nscene, const void *d_scenes, const int *d_scene_index,
+                              int enough_stable, const float *d_pose7, const float *d_joints, int nj, const int *joint_qposadr,
+                              int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg, uint8_t *d_labels, int *d_steps,
+                              void *stream);
+
 /* Batched mj_step on explicit states.  State record (state_stride reals, env-major):
  * qpos[nq] qvel[nv] qacc_warmstart[nv] ctrl[nu] mocap_pos[3] mocap_quat[4].  nstep = 0 runs
  * mj_forward only.  diag (may be NULL) receives diag_stride reals per env: header
@@ -116,7 +140,9 @@ int mgs_overflow_count(MgsModel *model);
 
 /* Per-candidate auxiliary results of the most recent launch on this model (synchronises the device): 4 floats per candidate -
  * [0] flags: bit 0 = the environment dropped contacts / constraint rows for lack of capacity (its label was computed on a
- *     truncated contact set: re-run it on a model created with larger capacities), bit 1 = the state blew up (label False);
+ *     truncated contact set: re-run it on a model created with larger capacities), bit 1 = the state blew up, or (clutter
+ *     scenes) the candidate's scene index was out of range (label False), bit 2 = skipped by the enough_stable early stop of
+ *     mgs_clutter_scenes_* (not simulated: its scene already had enough stable grasps; label False);
  * [1], [2] stability rollouts: displacement [m] and rotation [deg] of the grasped object over the close phase - what the
  *     reference computes as positional / rotational drift (mgs/env/gravityless_object_grasping.py:175-200) - NaN when the
  *     candidate lost contact before that point; [3] reserved (0). */

@@ -57,6 +57,8 @@ struct MgsModel {
   double qvel_clip;
   cudaStream_t stream;
   real *d_env_state;  // wide_g variant: the environments' state, one Layout.total slice per CTA of the persistent grid (else null)
+  unsigned int *d_scene_success;  // [scene_cap] successes per scene of the enough_stable early stop (grown on demand)
+  int scene_cap;
 };
 
 extern "C" const char *mgs_last_error(void) { return g_err.c_str(); }
@@ -222,6 +224,7 @@ extern "C" void mgs_model_destroy(MgsModel *M) {
   if (M->d_mpr_cache) cudaFree(M->d_mpr_cache);
   if (M->d_env_state) cudaFree(M->d_env_state);
   if (M->d_aux) cudaFree(M->d_aux);
+  if (M->d_scene_success) cudaFree(M->d_scene_success);
   if (M->d_stage) cudaFree(M->d_stage);
   if (M->h_stage) cudaFreeHost(M->h_stage);
   if (M->stream) cudaStreamDestroy(M->stream);
@@ -305,6 +308,7 @@ static int launch(MgsModel *M, const RolloutParams &prm, const BatchIO &io_in, c
     g_have_last[M->device] = 1;
   } else CU(cudaStreamWaitEvent(st, g_last_done[M->device], 0));
   CU(cudaMemsetAsync(M->d_counter, 0, 2 * sizeof(unsigned int), st));
+  if (io.scene_success) CU(cudaMemsetAsync(io.scene_success, 0, (size_t)io.nscene * sizeof(unsigned int), st));
   CU(M->ops->prepare(M->smem_per_block));
   KernelConsts kc;
   kc.m = M->dm; kc.L = M->L; kc.prm = prm; kc.io = io;
@@ -347,20 +351,43 @@ extern "C" int mgs_rollout_device(MgsModel *M, int mode, int n, const float *d_p
   return launch(M, prm, io, (cudaStream_t)stream);
 }
 
-extern "C" int mgs_clutter_device(MgsModel *M, int mode, int n, const void *d_scene, const float *d_pose7, const float *d_joints, int nj,
-                                  const int *joint_qposadr, int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg,
-                                  uint8_t *d_labels, int *d_steps, void *stream) {
+extern "C" int mgs_clutter_scenes_device(MgsModel *M, int mode, int n, int nscene, const void *d_scenes, const int *d_scene_index,
+                                         int enough_stable, const float *d_pose7, const float *d_joints, int nj, const int *joint_qposadr,
+                                         int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg, uint8_t *d_labels, int *d_steps,
+                                         void *stream) {
   if (!M) return fail("null model");
   if (mode != MGS_MODE_CLUTTER_COLLISION && mode != MGS_MODE_CLUTTER_STABLE) return fail("bad mode");
-  if (!d_scene) return fail("clutter rollouts need the scene state record");
+  if (!d_scenes) return fail("clutter rollouts need the scene state record");
+  if (nscene < 1) return fail("nscene must be >= 1");
   CU(cudaSetDevice(M->device));
   RolloutParams prm;
   if (fill_params(M, prm, mode, n, nj, joint_qposadr, base_qposadr, close_ctrl, cfg)) return -1;
   BatchIO io;
   memset(&io, 0, sizeof(io));
   io.pose7 = d_pose7; io.joints = d_joints; io.labels = d_labels; io.steps = d_steps;
-  io.state_in = (const real *)d_scene; io.state_stride = M->state_stride;
+  io.state_in = (const real *)d_scenes; io.state_stride = M->state_stride;
+  io.scene_index = d_scene_index; io.nscene = nscene;
+  if (enough_stable > 0 && n > 0) {  // the model's per-scene counters; launch() zeroes them on the launch stream
+    if (nscene > M->scene_cap) {
+      CU(cudaDeviceSynchronize());  // an earlier launch may still count into the old array
+      if (M->d_scene_success) cudaFree(M->d_scene_success);
+      M->d_scene_success = nullptr; M->scene_cap = 0;
+      const int cap = (nscene + 255) & ~255;
+      CU(cudaMalloc(&M->d_scene_success, (size_t)cap * sizeof(unsigned int)));
+      M->scene_cap = cap;
+    }
+    io.scene_success = M->d_scene_success;
+    io.enough_stable = enough_stable;
+  }
   return launch(M, prm, io, (cudaStream_t)stream);
+}
+
+// one scene, no index, no early stop
+extern "C" int mgs_clutter_device(MgsModel *M, int mode, int n, const void *d_scene, const float *d_pose7, const float *d_joints, int nj,
+                                  const int *joint_qposadr, int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg,
+                                  uint8_t *d_labels, int *d_steps, void *stream) {
+  return mgs_clutter_scenes_device(M, mode, n, 1, d_scene, nullptr, 0, d_pose7, d_joints, nj, joint_qposadr, base_qposadr, close_ctrl, cfg,
+                                   d_labels, d_steps, stream);
 }
 
 static int ensure_stage(MgsModel *M, size_t bytes) {
@@ -379,22 +406,29 @@ static size_t up256(size_t x) { return (x + 255) & ~size_t(255); }
 
 static int rollout_host(MgsModel *M, int mode, int n, const float *pose7, const float *joints, int nj, const int *joint_qposadr,
                         int base_qposadr, const double *close_ctrl, const MgsRolloutCfg *cfg, uint8_t *labels, int *steps,
-                        const double *scene = nullptr) {
+                        const double *scene = nullptr, int nscene = 1, const int *scene_index = nullptr, int enough_stable = 0) {
   if (!M) return fail("null model");
   if (n <= 0) return 0;
+  if (scene && nscene < 1) return fail("nscene must be >= 1");
+  if (scene_index)
+    for (int i = 0; i < n; i++)
+      if (scene_index[i] < 0 || scene_index[i] >= nscene) return fail("scene_index out of range [0, nscene)");
   CU(cudaSetDevice(M->device));
-  const size_t scene_bytes = scene ? (size_t)M->state_stride * sizeof(real) : 0;
+  const size_t scene_bytes = scene ? (size_t)nscene * M->state_stride * sizeof(real) : 0, index_bytes = scene_index ? (size_t)n * 4 : 0;
   size_t o_pose = 0, o_joint = up256(o_pose + (size_t)n * 7 * 4), o_scene = up256(o_joint + (size_t)n * (nj > 0 ? nj : 1) * 4),
-         o_lab = up256(o_scene + scene_bytes), o_steps = up256(o_lab + (size_t)n), total = up256(o_steps + (size_t)n * 4);
+         o_index = up256(o_scene + scene_bytes), o_lab = up256(o_index + index_bytes), o_steps = up256(o_lab + (size_t)n),
+         total = up256(o_steps + (size_t)n * 4);
   if (ensure_stage(M, total)) return -1;
   char *h = (char *)M->h_stage, *d = (char *)M->d_stage;
   memcpy(h + o_pose, pose7, (size_t)n * 7 * 4);
   memcpy(h + o_joint, joints, (size_t)n * nj * 4);
-  if (scene) { real *sr = (real *)(h + o_scene); for (int i = 0; i < M->state_stride; i++) sr[i] = (real)scene[i]; }
+  if (scene) { real *sr = (real *)(h + o_scene); for (size_t i = 0; i < (size_t)nscene * M->state_stride; i++) sr[i] = (real)scene[i]; }
+  if (scene_index) memcpy(h + o_index, scene_index, index_bytes);
   CU(cudaMemcpyAsync(d + o_pose, h + o_pose, o_lab, cudaMemcpyHostToDevice, M->stream));
   int rc;
-  if (scene) rc = mgs_clutter_device(M, mode, n, d + o_scene, (const float *)(d + o_pose), (const float *)(d + o_joint), nj, joint_qposadr,
-                                     base_qposadr, close_ctrl, cfg, (uint8_t *)(d + o_lab), (int *)(d + o_steps), M->stream);
+  if (scene) rc = mgs_clutter_scenes_device(M, mode, n, nscene, d + o_scene, scene_index ? (const int *)(d + o_index) : nullptr, enough_stable,
+                                            (const float *)(d + o_pose), (const float *)(d + o_joint), nj, joint_qposadr, base_qposadr,
+                                            close_ctrl, cfg, (uint8_t *)(d + o_lab), (int *)(d + o_steps), M->stream);
   else rc = mgs_rollout_device(M, mode, n, (const float *)(d + o_pose), (const float *)(d + o_joint), nj, joint_qposadr, base_qposadr,
                                close_ctrl, cfg, (uint8_t *)(d + o_lab), (int *)(d + o_steps), M->stream);
   if (rc) return rc;
@@ -428,6 +462,22 @@ extern "C" int mgs_clutter_stable_mask(MgsModel *M, int n, const double *scene, 
                                        uint8_t *stable_out, int *steps_out) {
   if (!scene) return fail("null scene");
   return rollout_host(M, MGS_MODE_CLUTTER_STABLE, n, pose7, joints, nj, joint_qposadr, base_qposadr, close_ctrl, cfg, stable_out, steps_out, scene);
+}
+
+extern "C" int mgs_clutter_scenes_collision_mask(MgsModel *M, int n, int nscene, const double *scenes, const int *scene_index,
+                                                 const float *pose7, const float *joints, int nj, const int *joint_qposadr, int base_qposadr,
+                                                 uint8_t *collision_free_out) {
+  if (!scenes || !scene_index) return fail("null scenes / scene_index");
+  return rollout_host(M, MGS_MODE_CLUTTER_COLLISION, n, pose7, joints, nj, joint_qposadr, base_qposadr, nullptr, nullptr, collision_free_out,
+                      nullptr, scenes, nscene, scene_index, 0);
+}
+
+extern "C" int mgs_clutter_scenes_stable_mask(MgsModel *M, int n, int nscene, const double *scenes, const int *scene_index, const float *pose7,
+                                              const float *joints, int nj, const int *joint_qposadr, int base_qposadr, int enough_stable,
+                                              const double *close_ctrl, const MgsRolloutCfg *cfg, uint8_t *stable_out, int *steps_out) {
+  if (!scenes || !scene_index) return fail("null scenes / scene_index");
+  return rollout_host(M, MGS_MODE_CLUTTER_STABLE, n, pose7, joints, nj, joint_qposadr, base_qposadr, close_ctrl, cfg, stable_out, steps_out,
+                      scenes, nscene, scene_index, enough_stable);
 }
 
 extern "C" int mgs_step_device(MgsModel *M, int n, int nstep, const void *d_state_in, void *d_state_out, void *d_diag_out, void *stream) {

@@ -238,4 +238,14 @@ struct BatchIO {
   // persistent grid - null for the variants that keep it in shared memory.  Last member: the constant-bank offsets of the fields
   // above stay where they were.
   real *env_state;
+  // Clutter modes over several scenes of one model (appended after env_state for the same reason).  Candidate i starts from the
+  // record state_in + scene_index[i] * state_stride; null = every candidate starts from scene 0 (nscene is then not read, so a
+  // zero-filled BatchIO behaves as before these members existed).  An index outside [0, nscene) gets label 0 and aux bit 1 without
+  // any read at that index.
+  const int *scene_index;  // [n]
+  int nscene;
+  // Device enough_stable early stop: non-overflowed successes per scene, counted during the launch; a candidate whose scene already
+  // counts >= enough_stable when it is pulled is not simulated (label 0, aux bit 2).  Null = no early stop.
+  unsigned int *scene_success;  // [nscene]
+  int enough_stable;
 };

@@ -171,8 +171,8 @@ MGS_DEVN void load_record_w(Env &e, const real *in) {
 
 // ClutterTableEnv.grasp_stable_mask body (clutter_table.py:288-317): restore the scene, place, close, lift with
 // the gripper-contact test at (t+1) % 100 == 0 (early break); label = lift survived
-MGS_DEVN int clutter_stable_program_w(Env &e, const float *pose7, const float *joints, int *steps) {
-  load_record_w(e, IO.state_in);
+MGS_DEVN int clutter_stable_program_w(Env &e, const real *scene, const float *pose7, const float *joints, int *steps) {
+  load_record_w(e, scene);
   place_w(e, pose7, joints);
   forward_w(e);
   MGS_STAGE_BARRIER(5);
@@ -270,22 +270,38 @@ MGS_DEVN void run_env_w(Env &e, int env) {
   const float *pose7 = IO.pose7 + (size_t)env * 7, *joints = IO.joints + (size_t)env * PRM.nj;
   float *aux = IO.aux ? IO.aux + 4 * (size_t)env : (float *)0;
   if (aux && MGS_LANE == 0) { aux[1] = nanf(""); aux[2] = nanf(""); aux[3] = 0; }
-  int label;
+  int label, skipped = 0;
+  const bool clutter = PRM.mode == MGS_MODE_CLUTTER_COLLISION || PRM.mode == MGS_MODE_CLUTTER_STABLE;
   if (PRM.mode == MGS_MODE_COLLISION) {
     reset_w(e);
     place_w(e, pose7, joints);
     forward_w(e);
     MGS_STAGE_BARRIER(5);
     label = (EH.ncon == 0);  // collision-free mask: no contact of any kind (check_contact, :306-307)
-  } else if (PRM.mode == MGS_MODE_CLUTTER_COLLISION) {
-    // ClutterTableEnv.grasp_collision_mask body (clutter_table.py:356-364); bounds test done by the host
-    load_record_w(e, IO.state_in);
-    place_w(e, pose7, joints);
-    forward_w(e);
-    MGS_STAGE_BARRIER(5);
-    label = !contact_with_object_w(e, 1);
-  } else if (PRM.mode == MGS_MODE_CLUTTER_STABLE) {
-    label = clutter_stable_program_w(e, pose7, joints, &steps);
+  } else if (clutter) {
+    // Scene of this candidate, and the enough_stable skip.  One thread decides (the one that pulls candidates and counts successes,
+    // so its next pull sees its own increment) and broadcasts: threads of the 256-thread variant that read the counter at different
+    // moments could otherwise disagree.  The counter is read with a volatile load, never through the read-only path.
+    const int s = IO.scene_index ? LDG(IO.scene_index + env) : 0;
+    int gate = 0;  // 0 = simulate, 1 = scene index out of range, 2 = skipped
+    if (IO.scene_index && (s < 0 || s >= IO.nscene)) gate = 1;  // no index array: scene 0, whatever nscene says
+    else if (IO.scene_success && MGS_LANE == 0 && *(volatile unsigned int *)(IO.scene_success + s) >= (unsigned int)IO.enough_stable) gate = 2;
+    gate = wbcasti(gate, 0);
+    const real *scene = IO.state_in + (size_t)(gate ? 0 : s) * IO.state_stride;
+    if (gate) {
+      EH.bad = gate == 1;
+      skipped = gate == 2;
+      label = 0;
+    } else if (PRM.mode == MGS_MODE_CLUTTER_COLLISION) {
+      // ClutterTableEnv.grasp_collision_mask body (clutter_table.py:356-364); bounds test done by the host
+      load_record_w(e, scene);
+      place_w(e, pose7, joints);
+      forward_w(e);
+      MGS_STAGE_BARRIER(5);
+      label = !contact_with_object_w(e, 1);
+    } else {
+      label = clutter_stable_program_w(e, scene, pose7, joints, &steps);
+    }
   } else {
     label = stability_program_w(e, pose7, joints, &steps, aux ? aux + 1 : (float *)0);
   }
@@ -293,10 +309,20 @@ MGS_DEVN void run_env_w(Env &e, int env) {
   PFOR(k, 1) {
     IO.labels[env] = (uint8_t)label;
     if (IO.steps) IO.steps[env] = steps;
-    if (aux) aux[0] = (float)((EH.overflow ? 1 : 0) | (EH.bad ? 2 : 0));
+    if (aux) aux[0] = (float)((EH.overflow ? 1 : 0) | (EH.bad ? 2 : 0) | (skipped ? 4 : 0));
 #ifndef MGS_HOST
     if (EH.overflow) atomicAdd(IO.work_counter + 1, 1u);
 #endif
+    // a success on the candidate's full contact set is final: count it for the early stop of its scene (the index is re-read here
+    // rather than kept live over the rollout)
+    if (clutter && IO.scene_success && label && !EH.overflow) {
+      const int s = IO.scene_index ? LDG(IO.scene_index + env) : 0;
+#ifdef MGS_HOST
+      IO.scene_success[s]++;
+#else
+      atomicAdd(IO.scene_success + s, 1u);
+#endif
+    }
   }
   if (IO.state_out) {
     real *out = IO.state_out + (size_t)env * IO.state_stride;

@@ -11,6 +11,7 @@ import subprocess
 
 import numpy as np
 
+from . import shard
 from .model_desc import MgsModelDesc, make_desc
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
@@ -99,6 +100,11 @@ def bind(L, prefix="mgs_"):
         L.mgs_step_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, vp]
         L.mgs_clutter_collision_mask.argtypes = [vp, C.c_int, dp, fp, fp, C.c_int, ip, C.c_int, u8p]
         L.mgs_clutter_stable_mask.argtypes = [vp, C.c_int, dp, fp, fp, C.c_int, ip, C.c_int, dp, C.POINTER(MgsRolloutCfg), u8p, ip]
+        L.mgs_clutter_scenes_collision_mask.argtypes = [vp, C.c_int, C.c_int, dp, ip, fp, fp, C.c_int, ip, C.c_int, u8p]
+        L.mgs_clutter_scenes_stable_mask.argtypes = [vp, C.c_int, C.c_int, dp, ip, fp, fp, C.c_int, ip, C.c_int, C.c_int, dp,
+                                                     C.POINTER(MgsRolloutCfg), u8p, ip]
+        L.mgs_clutter_scenes_device.argtypes = [vp, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp, vp, C.c_int, ip, C.c_int, dp,
+                                                C.POINTER(MgsRolloutCfg), vp, vp, vp]
         L.mgs_launch_count.restype = C.c_longlong
         L.mgs_overflow_count.argtypes = [vp]
         L.mgs_build_stamp.restype = C.c_char_p
@@ -159,6 +165,7 @@ class BatchSim:
         self.info = MgsModelInfo()
         self._check(self._f("model_info")(self.h, C.byref(self.info)))
         self.real = np.float32 if self.info.real_bytes == 4 else np.float64
+        self._order = None  # launch order of the most recent multi-scene call (last_aux maps its results back), else None
 
     def _f(self, name): return getattr(self.L, self.p + name)
 
@@ -235,6 +242,7 @@ class BatchSim:
         n = len(state)
         out = np.empty_like(state)
         diag = np.zeros((n, self.info.diag_stride), dtype=self.real) if want_diag else None
+        self._order = None
         self._check(self._f("step_host")(self.h, n, nstep, state.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
                                          diag.ctypes.data_as(C.c_void_p) if want_diag else None))
         return (out, self.unpack_diag(diag)) if want_diag else out
@@ -251,6 +259,7 @@ class BatchSim:
         pose7, joints, jadr = self._prep(pose7, joints, joint_qposadr)
         n = len(pose7)
         out = np.zeros(n, dtype=np.uint8)
+        self._order = None
         if self.p == "mgs_":
             rc = self.L.mgs_grasp_collision_mask(self.h, n, _fp(pose7), _fp(joints), joints.shape[1], _ip(jadr), int(base_qposadr), _u8(out))
         else:
@@ -264,6 +273,7 @@ class BatchSim:
         cc = np.ascontiguousarray(close_ctrl, dtype=np.float64)
         out = np.zeros(n, dtype=np.uint8)
         steps = np.zeros(n, dtype=np.int32)
+        self._order = None
         if self.p == "mgs_":
             rc = self.L.mgs_grasp_stability(self.h, n, _fp(pose7), _fp(joints), joints.shape[1], _ip(jadr), int(base_qposadr), _dp(cc),
                                             C.byref(cfg), _u8(out), _ip(steps))
@@ -279,6 +289,7 @@ class BatchSim:
         sc = np.ascontiguousarray(scene, dtype=np.float64)
         n = len(pose7)
         out = np.zeros(n, dtype=np.uint8)
+        self._order = None
         if n == 0:
             return out.astype(bool)
         if self.p == "mgs_":
@@ -295,6 +306,7 @@ class BatchSim:
         n = len(pose7)
         out = np.zeros(n, dtype=np.uint8)
         steps = np.zeros(n, dtype=np.int32)
+        self._order = None
         if n == 0:
             return out.astype(bool), steps
         if self.p == "mgs_":
@@ -306,14 +318,67 @@ class BatchSim:
         self._check(rc)
         return out.astype(bool), steps
 
+    def _clutter_scenes(self, mode, scenes, scene_index, pose7, joints, joint_qposadr, base_qposadr, close_ctrl, cfg, enough_stable):
+        pose7, joints, jadr = self._prep(pose7, joints, joint_qposadr)
+        n = len(pose7)
+        sc = np.ascontiguousarray(scenes, dtype=np.float64).reshape(-1, self.info.state_stride)
+        si = np.ascontiguousarray(scene_index, dtype=np.int32).reshape(-1)
+        if len(si) != n:
+            raise ValueError(f"scene_index has {len(si)} entries for {n} candidates")
+        out = np.zeros(n, dtype=np.uint8)
+        steps = np.zeros(n, dtype=np.int32)
+        self._order = None
+        if n == 0:
+            return out.astype(bool), steps
+        # round-robin across scenes, each scene's candidates in their own order: the device early stop is exact for that order
+        # and wastes only the candidates of a scene that are in flight when its count is reached
+        order = shard.scene_round_robin(si)
+        p7, jj, so = np.ascontiguousarray(pose7[order]), np.ascontiguousarray(joints[order]), np.ascontiguousarray(si[order])
+        lab, st = np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.int32)
+        cc = np.ascontiguousarray(close_ctrl if close_ctrl is not None else np.zeros(max(1, self.model.nu)), dtype=np.float64)
+        cfgp = C.byref(cfg) if cfg is not None else None
+        es = int(enough_stable or 0)
+        if self.p == "mgs_":
+            if mode == 3:
+                rc = self.L.mgs_clutter_scenes_collision_mask(self.h, n, len(sc), _dp(sc), _ip(so), _fp(p7), _fp(jj), jj.shape[1], _ip(jadr),
+                                                              int(base_qposadr), _u8(lab))
+            else:
+                rc = self.L.mgs_clutter_scenes_stable_mask(self.h, n, len(sc), _dp(sc), _ip(so), _fp(p7), _fp(jj), jj.shape[1], _ip(jadr),
+                                                           int(base_qposadr), es, _dp(cc), cfgp, _u8(lab), _ip(st))
+        else:
+            rc = self.L.l1_clutter_scenes_host(self.h, mode, n, len(sc), _dp(sc), _ip(so), es if mode == 4 else 0, _fp(p7), _fp(jj),
+                                               jj.shape[1], _ip(jadr), int(base_qposadr), _dp(cc), cfgp, _u8(lab), _ip(st))
+        self._check(rc)
+        self._order = order
+        out[order], steps[order] = lab, st
+        return out.astype(bool), steps
+
+    def clutter_scenes_collision_mask(self, scenes, scene_index, pose7, joints, joint_qposadr, base_qposadr):
+        """clutter_collision_mask over several scenes of this model in one launch: `scenes` [nscene][state_stride] records, candidate i
+        starts from scenes[scene_index[i]]."""
+        return self._clutter_scenes(3, scenes, scene_index, pose7, joints, joint_qposadr, base_qposadr, None, None, 0)[0]
+
+    def clutter_scenes_stable_mask(self, scenes, scene_index, pose7, joints, joint_qposadr, base_qposadr, close_ctrl, cfg: MgsRolloutCfg,
+                                   enough_stable: int = 0):
+        """clutter_stable_mask over several scenes in one launch -> (labels bool[n], steps int32[n]).  enough_stable > 0: a candidate
+        whose scene already had that many non-overflowed successes when it was pulled is not simulated (label False, last_aux
+        `skipped`); the per-scene prefix rule (shard.apply_enough_stable) is left to the caller."""
+        return self._clutter_scenes(4, scenes, scene_index, pose7, joints, joint_qposadr, base_qposadr, close_ctrl, cfg, enough_stable)
+
     def last_aux(self, n: int):
-        """Per-candidate auxiliary results of the most recent launch: dict(overflow bool[n], bad bool[n], pos_drift f32[n],
-        rot_drift_deg f32[n]) - see mgs_last_aux in include/mgs_b200.h."""
+        """Per-candidate auxiliary results of the most recent launch: dict(overflow bool[n], bad bool[n], skipped bool[n],
+        pos_drift f32[n], rot_drift_deg f32[n]) - see mgs_last_aux in include/mgs_b200.h.  After a multi-scene call they are in
+        the caller's candidate order."""
         a = np.zeros((n, 4), dtype=np.float32)
         if n:
             self._check(self._f("last_aux")(self.h, n, _fp(a)))
+        if self._order is not None and len(self._order) == n:
+            b = np.empty_like(a)
+            b[self._order] = a
+            a = b
         fl = a[:, 0].astype(np.int32)
-        return dict(overflow=(fl & 1).astype(bool), bad=(fl & 2).astype(bool), pos_drift=a[:, 1].copy(), rot_drift_deg=a[:, 2].copy())
+        return dict(overflow=(fl & 1).astype(bool), bad=(fl & 2).astype(bool), skipped=(fl & 4).astype(bool), pos_drift=a[:, 1].copy(),
+                    rot_drift_deg=a[:, 2].copy())
 
     def set_qvel_clip(self, clip: float):
         """step(): clamp qvel to +-clip before every step (scene generation); 0 = off."""
@@ -331,6 +396,7 @@ class BatchSim:
         """Device-pointer variant (torch tensors' .data_ptr()); asynchronous on `stream_ptr`."""
         jadr = np.ascontiguousarray(joint_qposadr, dtype=np.int32)
         cc = np.ascontiguousarray(close_ctrl if close_ctrl is not None else np.zeros(max(1, self.model.nu)), dtype=np.float64)
+        self._order = None
         self._check(self.L.mgs_rollout_device(self.h, mode, n, d_pose7_ptr, d_joints_ptr, nj, _ip(jadr), int(base_qposadr), _dp(cc),
                                               C.byref(cfg) if cfg is not None else None, d_labels_ptr, d_steps_ptr, stream_ptr))
 

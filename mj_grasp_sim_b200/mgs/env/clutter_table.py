@@ -16,7 +16,7 @@ import numpy as np
 from ... import scenes
 from ...compiler.mjcf import compile_mjcf
 from ...lib import BatchSim, MgsRolloutCfg
-from ...shard import evaluate_sharded
+from ...shard import apply_enough_stable, evaluate_sharded
 from ..core.simualtion import MjSimulation
 from .gravityless_object_grasping import EscalatingSim
 from ..util.geo.transforms import SE3Pose
@@ -101,6 +101,28 @@ class ClutterTableEnv(MjSimulation):
                 continue
             self._record, self._time = recs[k], 11.7
             out.append(self.to_dict())
+        self._record, self._time = keep_rec, keep_time
+        return out
+
+    def gen_clutter_scenes(self, seeds):
+        """Scene k = what gen_clutter(seeds[k]) followed by to_dict() makes on this environment (state time included), for all
+        seeds in one batch of launches; None where is_stable() would then be False."""
+        info = dict(base_qposadr=self.gripper.get_freejoint_idxs(self)[0],
+                    object_qposadr=[int(self.model.jnt_qposadr[self.model.names["joint"][f"{n}:joint"]]) for n in self.object_names])
+        step = lambda r, k: self.sim.step(r.astype(self.sim.real), k).astype(np.float64)
+        self.sim.set_qvel_clip(50.0)
+        try:
+            recs = scenes.gen_clutter_batch(self.model, info, step, seeds)
+        finally:
+            self.sim.set_qvel_clip(0.0)
+        ok, _ = scenes.scenes_stable(self.model, info, step, recs.copy())
+        t = self._time
+        for _ in range(9 * len(self.object_names) + 90):  # gen_clutter advances the time in steps of 100 (_step)
+            t += 100 * float(self.model.opt["timestep"])
+        out, keep_rec, keep_time = [], self._record, self._time
+        for k in range(len(recs)):
+            self._record, self._time = recs[k], t
+            out.append(self.to_dict() if ok[k] else None)
         self._record, self._time = keep_rec, keep_time
         return out
 
@@ -194,6 +216,57 @@ class ClutterTableEnv(MjSimulation):
         # enough_stable as the reference's early stop (:293-296), in rounds of one GPU-filling chunk per rank
         info = self.sim.info
         return evaluate_sharded(len(pose7), run_range, enough_stable, chunk=info.warps_per_block * info.blocks_per_sm * info.num_sms)
+
+    # ---- many scenes of this model in one launch ----------------------------------------------------
+    def _scene_records(self, env_states):
+        return np.stack([self._record_from_state(s) for s in env_states]) if len(env_states) else np.zeros((0, self.sim.info.state_stride))
+
+    def grasp_collision_mask_scenes(self, poses: SE3Pose, joints: np.ndarray, scene_index, env_states):
+        """grasp_collision_mask for candidates of several scenes of this model (same gripper, objects and masks) in one launch:
+        candidate i is tested in the scene env_states[scene_index[i]] (mjSTATE_INTEGRATION vectors).  Equals grasp_collision_mask
+        called per scene with that scene's state set."""
+        pose7, j32, jadr = self._process(poses, joints)
+        si = np.asarray(scene_index, dtype=np.int64).reshape(-1)
+        if len(si) != len(pose7):
+            raise ValueError(f"scene_index has {len(si)} entries for {len(pose7)} candidates")
+        recs = self._scene_records(env_states)
+        p = np.asarray(poses.pos).reshape(-1, 3)
+        in_bound = (p[:, 0] < 0.25) & (p[:, 0] > -0.25) & (p[:, 1] < 0.25) & (p[:, 1] > -0.25) & (p[:, 2] < 1.0) & (p[:, 2] > 0.0)  # :344-354
+        out = np.zeros(len(pose7), dtype=bool)
+        idx = np.nonzero(in_bound)[0]
+        base = self.gripper.get_freejoint_idxs(self)[0]
+        if len(idx):
+            p7, jj, s = pose7[idx], j32[idx], si[idx]
+            sel = lambda k: (s, p7, jj) if k is None else (s[k], p7[k], jj[k])
+            out[idx] = self._esc.run(lambda sim, k: sim.clutter_scenes_collision_mask(recs, *sel(k), jadr, base), len(idx))[0]
+        return out
+
+    def grasp_stable_mask_scenes(self, poses: SE3Pose, joints: np.ndarray, scene_index, env_states, nstep_lift: int = 3000, lift_dist: float = 0.3,
+                                 enough_stable=None):
+        """grasp_stable_mask for candidates of several scenes of this model in one launch; candidate i starts from
+        env_states[scene_index[i]], and each scene's candidates are taken in their order here.  `enough_stable` applies per scene,
+        as the early stop of the device (include/mgs_b200.h, mgs_clutter_scenes_*): the result equals grasp_stable_mask called once
+        per scene with the same enough_stable.  Overflowed candidates are re-run up the capacity ladder without the early stop."""
+        pose7, j32, jadr = self._process(poses, joints)
+        si = np.asarray(scene_index, dtype=np.int64).reshape(-1)
+        if len(si) != len(pose7):
+            raise ValueError(f"scene_index has {len(si)} entries for {len(pose7)} candidates")
+        recs = self._scene_records(env_states)
+        base = self.gripper.get_freejoint_idxs(self)[0]
+        cfg = MgsRolloutCfg(self.gripper.NSTEP_CLOSE, nstep_lift, 0, self.gripper.REPOSE_ON_CLOSE, lift_dist, 0.0)
+        ctrl = self.gripper.close_ctrl()
+        es = int(enough_stable) if enough_stable is not None else 0
+
+        def call(sim, k):
+            if k is None:
+                return sim.clutter_scenes_stable_mask(recs, si, pose7, j32, jadr, base, ctrl, cfg, enough_stable=es)
+            return sim.clutter_scenes_stable_mask(recs, si[k], pose7[k], j32[k], jadr, base, ctrl, cfg, enough_stable=0)
+        lab = np.asarray(self._esc.run(call, len(pose7))[0][0], dtype=bool)
+        if enough_stable is not None:
+            for s in np.unique(si):
+                rows = si == s
+                lab[rows] = apply_enough_stable(lab[rows], enough_stable)
+        return lab
 
     # ---- persistence (scene.npz payload) --------------------------------------------------------
     def to_dict(self):

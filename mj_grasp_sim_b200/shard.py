@@ -88,3 +88,51 @@ def evaluate_sharded(n: int, run_range, enough_stable=None, chunk: int = 0) -> n
         count += int(got.sum())
         done += rn
     return apply_enough_stable(labels, enough_stable)
+
+
+def scene_round_robin(scene_index) -> np.ndarray:
+    """Launch order for candidates of several scenes: the first candidate of every scene (in scene order), then the second of
+    every scene, and so on.  Each scene's own candidates keep their order, which is what the device enough_stable early stop
+    needs (include/mgs_b200.h, mgs_clutter_scenes_*).  Returns `order` (launch position j runs candidate order[j]); results
+    come back with `out[order] = launched`."""
+    s = np.asarray(scene_index, dtype=np.int64).reshape(-1)
+    if not len(s):
+        return np.zeros(0, dtype=np.int64)
+    by_scene = np.argsort(s, kind="stable")
+    first = np.concatenate([[0], np.nonzero(np.diff(s[by_scene]))[0] + 1])
+    rank = np.empty(len(s), dtype=np.int64)
+    rank[by_scene] = np.arange(len(s)) - np.repeat(first, np.diff(np.concatenate([first, [len(s)]])))
+    return np.lexsort((s, rank))
+
+
+def plan_scenes(counts, world: int) -> list:
+    """Whole scenes per rank, balanced by candidate count (longest-processing-time first; ties to the lower rank).  Returns per-rank
+    sorted lists of scene indices."""
+    load = [0] * world
+    plan = [[] for _ in range(world)]
+    for s in sorted(range(len(counts)), key=lambda s: (-int(counts[s]), s)):
+        r = min(range(world), key=lambda r: (load[r], r))
+        plan[r].append(s)
+        load[r] += int(counts[s])
+    return [sorted(p) for p in plan]
+
+
+def evaluate_scenes_sharded(scene_index, nscene: int, run_scenes) -> np.ndarray:
+    """Labels bool[n] of candidates of several scenes, each rank evaluating whole scenes: `run_scenes(candidates) -> bool[len]` runs the
+    given candidate indices (in increasing order, all of this rank's scenes) on this rank's GPU.  A scene's enough_stable early stop
+    never crosses ranks this way.  The labels are combined by one MAX all-reduce of the full uint8 array (every candidate is
+    written by exactly one rank), as mixed.run_mixed does."""
+    s = np.asarray(scene_index, dtype=np.int64).reshape(-1)
+    world, rank, dev = dist_state()
+    if world == 1:
+        return np.asarray(run_scenes(np.arange(len(s))), dtype=bool)
+    mine = plan_scenes(np.bincount(s, minlength=nscene), world)[rank]
+    idx = np.nonzero(np.isin(s, mine))[0]
+    local = np.zeros(len(s), dtype=np.uint8)
+    if len(idx):
+        local[idx] = np.asarray(run_scenes(idx), dtype=np.uint8)
+    import torch
+    import torch.distributed as dist
+    flat = torch.as_tensor(local, device=dev)
+    dist.all_reduce(flat, op=dist.ReduceOp.MAX)
+    return flat.cpu().numpy().astype(bool)
